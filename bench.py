@@ -41,6 +41,10 @@ WORKLOADS = {
 DEFAULT_WORKLOAD = "newref_600x50kb"
 METRIC = "newref_bin_pairs_per_s"
 UNIT = "bin-pairs/s"
+# --dump-outputs: the search table and the test path's per-bin vectors, sampled to these sizes in float64 (with the test
+# batch's chromosome-wide z-scores, sigma averages and calls the dump stays below 64 MB)
+DUMP_TABLE_BYTES = 40 * 10**6
+DUMP_TEST_BYTES = 16 * 10**6
 
 
 def pairs_for_rows(bins, r0, r1):
@@ -51,6 +55,35 @@ def pairs_for_rows(bins, r0, r1):
 
 def get_part(partnum, outof, bincount):
     return int(bincount / float(outof) * partnum), int(bincount / float(outof) * (partnum + 1))
+
+
+def _sample_rows(n, keep):
+    """All of range(n), or `keep` of them drawn with a fixed seed: two builds dump the same rows."""
+    return np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+
+
+def dump_outputs(path, table_idx, table_dist):
+    """The reference-bin table (what a reference npz stores as `indexes` / `distances`) as float64 .npy files."""
+    n, k = table_idx.shape
+    rows = _sample_rows(n, DUMP_TABLE_BYTES // (16 * k))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "indexes.npy"), table_idx.cpu().numpy()[rows].astype(np.float64))
+    np.save(os.path.join(path, "distances.npy"), table_dist.cpu().numpy()[rows])
+
+
+def dump_test_outputs(path, z, r, asdef, cwz, calls):
+    """One test batch's results (what a result npz stores per sample) as float64 .npy files: z-scores and ratios of a
+    sample of the batch's samples, and the chromosome-wide z-scores, sigma averages and calls (sample, chromosome,
+    start bin, end bin, z) of all of them."""
+    b, n = z.shape
+    samples = _sample_rows(b, max(1, DUMP_TEST_BYTES // (16 * n)))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "test_z.npy"), z.cpu().numpy()[samples])
+    np.save(os.path.join(path, "test_r.npy"), r.cpu().numpy()[samples])
+    np.save(os.path.join(path, "test_asdef.npy"), asdef.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(path, "test_cwz.npy"), cwz.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(path, "test_calls.npy"),
+            np.stack([calls[f].astype(np.float64) for f in ("sample", "chrom", "x", "y", "z")], axis=1).reshape(-1, 5))
 
 
 def fp64_peak():
@@ -314,6 +347,7 @@ def bench_test_path(args, torch, dist, device, dev, rank, world, local, X, bins,
     host_n = torch.empty((B, n), dtype=torch.int32).pin_memory()
 
     copy_out = torch.cuda.Stream(device=dev)
+    last = {}               # --dump-outputs: the results of the latest batch
     in_flight = []          # (device tensors, copy-finished event) of the batches whose results are still travelling
 
     host_cwz = torch.empty((B, 22), dtype=torch.float64).pin_memory()
@@ -324,6 +358,8 @@ def bench_test_path(args, torch, dist, device, dev, rank, world, local, X, bins,
         T = device.test_prep(counts, masked_raw, mean, comps)
         z, r, sizes, asdef = device.zscore_batch(T, B, table, thr, 5)
         cwz, cleaned, calls = device.segment_batch(z, sizes, bins, list(range(22)), 25, thr, 3)   # calls: on the host already
+        if args.dump_outputs:
+            last.update(z=z, r=r, asdef=asdef, cwz=cwz, calls=calls)
         if from_host and not full:      # compact result: calls, chromosome-wide z, sigma average (what a report needs)
             host_cwz.copy_(torch.as_tensor(cwz).reshape(B, -1)[:, :22], non_blocking=True)
             host_sd.copy_(torch.as_tensor(asdef).reshape(-1)[:B], non_blocking=True)
@@ -346,7 +382,7 @@ def bench_test_path(args, torch, dist, device, dev, rank, world, local, X, bins,
     for _ in range(2):
         ncalls = run(False)
     torch.cuda.synchronize(dev)
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     zs, sg, pr, executed = [], [], [], []
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     if world > 1:
@@ -360,8 +396,10 @@ def bench_test_path(args, torch, dist, device, dev, rank, world, local, X, bins,
         executed.append(st["zscore_pairs_per_pass"])
     e1.record()
     torch.cuda.synchronize(dev)
+    if args.dump_outputs and rank == 0:
+        dump_test_outputs(args.dump_outputs, **last)
     dev_ms = e0.elapsed_time(e1) / steps
-    e2e_steps = max(steps, 4)
+    e2e_steps = steps
     e2e_both = []
     for full in (False, True):
         run(True, full)
@@ -520,7 +558,13 @@ def main():
                     help="N > 1: getPart row shards + all-gather (default), or the sharded symmetric search")
     ap.add_argument("--no-parity-check", action="store_true", help="skip the sampled-row comparison with the C oracle")
     ap.add_argument("--test-batch", type=int, default=512, help="test samples per GPU in the test section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as float64 .npy files: the reference-bin table "
+                         "(DIR/indexes.npy, DIR/distances.npy) and the test section's batch (DIR/test_*.npy); larger outputs "
+                         "keep a fixed seeded sample of rows, under 64 MB in all (bench_outputs/ is git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -649,7 +693,7 @@ def main():
     if big:
         e2e = None      # validation-only workload: the matrix never exists on the host
     else:
-        e2e_steps = max(2, min(args.steps, 5))
+        e2e_steps = args.steps
         if world > 1:
             # every rank uploads 1/N of the matrix, NCCL all-gathers it over NVLink, searches its rows, copies them back
             sharded = shard.ShardedSearch(n, S, k, rank, world, dev, symmetric=sym_search is not None)
@@ -793,6 +837,8 @@ def main():
         table_idx, table_dist = out_idx[:rows], out_dist[:rows]
     else:
         table_idx, table_dist = full_idx, full_dist
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, table_idx, table_dist)
     pc = None
     if not args.no_parity_check:
         pc = parity_check(device, torch, X, X_host_np, bins, k, table_idx, table_dist, rank, world, local,

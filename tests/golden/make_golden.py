@@ -278,6 +278,81 @@ def golden_segmin_nonfinite():
     np.savez_compressed(os.path.join(HERE, "segmin_nonfinite.npz"), **out)
 
 
+def search_case(seed):
+    """(bins, X, k) of tests/test_oracle_vs_ref.py::test_search_random: 2-6 chromosomes of 1-24 bins, 1-39 samples, k up
+    to 29 (often more than a chromosome's candidates) and one duplicated row."""
+    rng = np.random.default_rng(seed)
+    bins = [int(b) for b in rng.integers(1, 25, size=int(rng.integers(2, 7)))]
+    n, S, k = sum(bins), int(rng.integers(1, 40)), int(rng.integers(1, 30))
+    X = 1.0 + rng.normal(0, 0.05, size=(n, S))
+    X[rng.integers(0, n)] = X[rng.integers(0, n)]
+    return bins, X, k
+
+
+def zscore_case(seed):
+    """(bins, X, test) of test_zscores_random; the search table is wc_oracle.get_reference(X, bins, sums, 9, 1, 1)."""
+    rng = np.random.default_rng(100 + seed)
+    bins = [int(b) for b in rng.integers(5, 30, size=4)]
+    n = sum(bins)
+    X = 1.0 + rng.normal(0, 0.05, size=(n, 10))
+    test = 1.0 + rng.normal(0, 0.03, size=n)
+    test[3:9] *= 1.3
+    return bins, X, test
+
+
+def segmentation_case(seed):
+    """z of test_segmentation_random: 1-159 bins, one shifted run when there are more than 20."""
+    rng = np.random.default_rng(200 + seed)
+    n = int(rng.integers(1, 160))
+    z = rng.normal(0, 1, size=n)
+    if n > 20:
+        a = int(rng.integers(0, n - 10))
+        z[a:a + int(rng.integers(2, 10))] += rng.choice([-2.0, 2.0])
+    return z
+
+
+RANDOM_SEEDS = {"search": range(4), "zscores": range(3), "segmentation": range(4)}
+
+
+def reference_random_outputs(ref_wt):
+    """The reference's outputs on the seeded cases above: getReference, getOptimalCutoff + repeatTest(2.5, 4) on the
+    oracle's table, fillTri + segmentTri(3.0, 3).  `ref_wt` is the reference's wisetools module."""
+    import wc_oracle
+    out = {}
+    for seed in RANDOM_SEEDS["search"]:
+        bins, X, k = search_case(seed)
+        with contextlib.redirect_stdout(io.StringIO()):
+            out["search%d_idx" % seed], out["search%d_dst" % seed] = ref_wt.getReference(
+                np.asfortranarray(X), bins, list(np.cumsum(bins)), k, 1, 1)
+    for seed in RANDOM_SEEDS["zscores"]:
+        bins, X, test = zscore_case(seed)
+        sums = list(np.cumsum(bins))
+        idx, dst = wc_oracle.get_reference(X, bins, sums, 9, 1, 1)
+        cutoff, _ = ref_wt.getOptimalCutoff(dst, 3)
+        with contextlib.redirect_stdout(io.StringIO()):
+            z, r, sizes, sd = ref_wt.repeatTest(np.copy(test), idx, dst, bins, sums, cutoff, 2.5, 4)
+        out.update({"zscores%d_cutoff" % seed: cutoff, "zscores%d_z" % seed: z, "zscores%d_r" % seed: r,
+                    "zscores%d_sizes" % seed: sizes, "zscores%d_sd" % seed: sd})
+    for seed in RANDOM_SEEDS["segmentation"]:
+        z = segmentation_case(seed)
+        tri = ref_wt.fillTri(z)
+        out["segmentation%d_cw" % seed] = tri.getValue(0, len(z) - 1)
+        out["segmentation%d_calls" % seed] = np.array([[x, y, v] for v, (x, y) in tri.segmentTri(3.0, 3)],
+                                                      dtype=float).reshape(-1, 3)
+    return out
+
+
+def golden_oracle_random():
+    """reference_random_outputs of the reference itself, for tests/test_oracle_vs_ref.py where oracle/_ref is absent."""
+    sys.path.insert(0, REF)
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    with contextlib.redirect_stdout(io.StringIO()):
+        import wisetools as ref_wt
+    out = reference_random_outputs(ref_wt)
+    np.savez_compressed(os.path.join(HERE, "oracle_random.npz"), **out)
+    print("oracle_random.npz: %d arrays" % len(out))
+
+
 def golden_cli_tiny_mineff():
     """The reference's `test -mineffectsize` (wisecondor.py:460, fillTriMin) on the tiny genome's test samples against the
     reference npz of tiny_cli.npz (rebuilt from its arrays, as tests/test_cli_gpu.py does): 0.25 keeps the 1.3x gain of
@@ -403,6 +478,9 @@ def main():
     if '--segmin-only' in sys.argv:
         golden_segmin_nonfinite()
         return 0
+    if '--random-only' in sys.argv:
+        golden_oracle_random()
+        return 0
     golden_functions()
     golden_cli_tiny()
     golden_report()
@@ -410,6 +488,7 @@ def main():
     golden_cli_tiny_mineff()
     golden_cli_tiny_flags()
     golden_cli_tiny_prep_binsize()
+    golden_oracle_random()
     return 0
 
 

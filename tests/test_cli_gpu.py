@@ -363,6 +363,29 @@ def test_parts_interchangeable_with_the_reference_workers(workdir, tiny):
         assert np.array_equal(mixed[key], whole[key]), key
 
 
+def test_parts_on_the_reference_prep_file_match_reference(workdir, tiny):
+    """This build's `newrefpart` and `newrefpost` on the prep file the reference's own `newrefprep` wrote (rebuilt from its
+    arrays in tests/golden/tiny_cli.npz): part 2 of 3 holds bit for bit the reference's rows of that part, and the
+    assembled reference file equals the one the reference's `newrefpost` wrote from its three parts."""
+    prep = str(workdir / "goldprep.npz")
+    np.savez_compressed(prep, arguments={}, runtime={}, binsize=tiny['binsize'], chromosomeBins=tiny['ref_chromosome_sizes'],
+                        maskedData=tiny['prep_maskedData'], mask=tiny['prep_mask'],
+                        maskedChromBins=tiny['prep_maskedChromBins'], maskedChromBinSums=tiny['prep_maskedChromBinSums'],
+                        correctedData=np.asfortranarray(tiny['prep_correctedData']),
+                        pca_components=tiny['ref_pca_components'], pca_mean=tiny['ref_pca_mean'])
+    for part in (1, 2, 3):
+        _run(["newrefpart", prep, str(workdir / "gold_part"), str(part), "3", "-refsize", "40"])
+    a, b = wc_oracle.get_part(1, 3, tiny['ref_indexes'].shape[0])
+    mine = np.load(str(workdir / "gold_part_2.npz"), allow_pickle=True)
+    assert np.array_equal(mine['indexes'], tiny['ref_indexes'][a:b])
+    assert np.array_equal(mine['distances'], tiny['ref_distances'][a:b])
+    _run(["newrefpost", prep, str(workdir / "gold_part"), "3", str(workdir / "gold.npz")])
+    r = np.load(str(workdir / "gold.npz"), allow_pickle=True)
+    for key in ("indexes", "distances", "chromosome_sizes", "mask", "masked_sizes", "pca_mean", "pca_components"):
+        assert np.array_equal(r[key], tiny['ref_' + key]), key
+    assert r['binsize'].item() == tiny['ref_binsize'].item()
+
+
 def test_reference_consumers_read_our_results(workdir, tiny):
     """The reference's own `report` tool (a pure consumer of sample + result npz, wisecondor.py:304-342) and its `test`
     tool accept the files this build writes."""
