@@ -407,6 +407,69 @@ def segment_region_prefix(region, threshold, min_search=3):
     return cw, rec(0, n)
 
 
+def segment_region_exact(region, threshold, min_search=3, max_window=10 ** 6):
+    """segment_region's result, bit for bit, for finite z at chromosome sizes (5 000 - 25 000 bins) where
+    fill_triangle's O(n^3) loop is out of reach.
+
+    Per pending range [lo, hi) the runs are located with fp64 prefix sums of region[lo:hi] (rebased per range), one
+    vectorised row x at a time.  Every run whose located |value| is within `tol` of the located maximum M is kept, with
+    tol = 4 m eps sum|region[lo:hi]| + 8 eps M: each prefix end and numpy's own pairwise sum are off by at most
+    m eps sum|z|, the subtraction, 1/sqrt and product by a few eps |value|.  Those runs alone are re-scored exactly
+    as the reference does (np.sum(region[x:y+1]) / np.sqrt(y-x+1), wisetools.py:471) and the reference's rules decide:
+    max, then min, abs(min) > max, first occurrence in row-major order, threshold, recursion (triarray.py:59-84).  A
+    window of more than `max_window` runs raises instead of guessing."""
+    z = np.asarray(region, dtype=np.float64)
+    n = z.shape[0]
+    if n == 0:
+        raise ValueError("empty region")
+    if not np.isfinite(z).all():
+        raise ValueError("segment_region_exact takes finite z only")
+    eps = np.finfo(np.float64).eps
+    inv = 1.0 / np.sqrt(np.arange(1, n + 1, dtype=np.float64))
+
+    def champion(lo, hi):
+        m = hi - lo
+        p = np.concatenate(([0.0], np.cumsum(z[lo:hi])))
+        rowmax = np.empty(m)
+        for x in range(m):
+            rowmax[x] = np.max(np.abs((p[x + 1:] - p[x]) * inv[:m - x]))
+        big = float(np.max(rowmax))
+        tol = 4.0 * m * eps * float(np.sum(np.abs(z[lo:hi]))) + 8.0 * eps * big
+        if big + tol < threshold:                             # every |value| is below the threshold: no call
+            return None
+        floor = big - 2.0 * tol
+        cands = []
+        for x in np.flatnonzero(rowmax >= floor):
+            ys = np.flatnonzero(np.abs((p[x + 1:] - p[x]) * inv[:m - x]) >= floor)
+            cands.extend((lo + int(x), lo + int(x) + int(j)) for j in ys)
+            if len(cands) > max_window:
+                raise ValueError("segment_region_exact: more than %d runs within %g of the maximum" % (max_window, tol))
+        best_max = best_min = None
+        for x, y in cands:                                    # row-major order: strict comparisons keep the first
+            v = np.sum(z[x:y + 1]) / np.sqrt(y - x + 1)
+            if best_max is None or v > best_max[0]:
+                best_max = (v, x, y)
+            if best_min is None or v < best_min[0]:
+                best_min = (v, x, y)
+        return best_min if abs(best_min[0]) > best_max[0] else best_max
+
+    calls = []
+    pending = [(0, n)]
+    while pending:
+        lo, hi = pending.pop()
+        best = champion(lo, hi)
+        if best is None or abs(best[0]) < threshold:
+            continue
+        v, x, y = best
+        calls.append((v, (x, y)))
+        if x - lo > min_search:
+            pending.append((lo, x))
+        if (y - lo) + 1 < (hi - lo) - min_search:
+            pending.append((y + 1, hi))
+    calls.sort(key=lambda c: c[1][0])                         # the reference's in-order recursion: left, call, right
+    return np.sum(z) / np.sqrt(n), calls
+
+
 # --------------------------------------------------------------------------------------------------------
 # test driver                                                                  wisecondor.py:174-281
 # --------------------------------------------------------------------------------------------------------

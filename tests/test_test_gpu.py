@@ -284,7 +284,8 @@ def test_segmentation_min_effect_non_finite_golden_and_random():
 
 
 def test_segmentation_very_long_chromosome_uses_global_side_arrays():
-    """chr1 at 10 kb bins has 24 926 bins: the prefix sums alone fill shared memory, the side arrays move to global."""
+    """A chromosome of 20 000 bins, about chr1 at 10 kb bins (24 926): prefix sums and side arrays take 160 KB of
+    shared memory."""
     rng = np.random.default_rng(8)
     n = 20000
     z = rng.normal(0, 1, size=n)

@@ -45,7 +45,7 @@ enum {
     SLOT_XC = 0, SLOT_NORMS, SLOT_ROWCS, SLOT_ROWCE, SLOT_RBMETA, SLOT_CAND_D, SLOT_CAND_J, SLOT_SEGCNT,
     SLOT_SEGFLAG, SLOT_SLOW, SLOT_SCRATCH, SLOT_IO_X, SLOT_IO_IDX, SLOT_IO_DIST, SLOT_ROWTHR,
     SLOT_IN_KEY, SLOT_IN_J, SLOT_IN_CNT, SLOT_N32, SLOT_F16STAT,                                                             // search
-    SLOT_PROF = 20, SLOT_PIV_IDS = 21, SLOT_PIV_X = 22, SLOT_PIV_N = 23, SLOT_PIV_META = 37,
+    SLOT_PROF = 20, SLOT_PIV_IDS = 21, SLOT_PIV_X = 22, SLOT_PIV_N = 23, SLOT_PIV_META = 37, SLOT_S_STACK = 38,
     SLOT_T_COPY = 24, SLOT_T_ZT, SLOT_T_RT, SLOT_T_NT, SLOT_T_SD, SLOT_T_FLAGS, SLOT_T_TOTALS, SLOT_T_PROJ,   // test
     SLOT_T_REVCNT = 44, SLOT_T_REVCUR, SLOT_T_DIRTY, SLOT_T_PAIRS,
     SLOT_S_ZC = 32, SLOT_S_META, SLOT_S_STATUS, SLOT_S_RC, SLOT_S_AUX,                                                       // segmentation

@@ -27,9 +27,9 @@ constexpr int SEG_THREADS = 128;
 constexpr int SEG_WARPS = SEG_THREADS / 32;
 constexpr int SEG_R = 5;                      // run lengths per lane in the sweep (odd: conflict-free prefix reads)
 constexpr int SEG_TILE = 32 * SEG_R;          // run lengths per warp tile
-constexpr int SEG_STACK = 128;                // pending ranges per chromosome
 constexpr int SEG_ROWCAP = 1024;              // diagonals re-scored exactly per search before falling back to all of them
 constexpr double SEG_EPS = 1.1102230246251565e-16;
+constexpr double SEG_FLT_TINY = 8.0 * 1.1754943508222875e-38;   // 8 x FLT_MIN: flush / subnormal rounding of the fp32 sweep
 
 struct SegArgs {
     const double* z;         // [B][N]
@@ -38,6 +38,7 @@ struct SegArgs {
     const int* sel_start;    // [nsel] first masked bin of each selected chromosome (sorted by descending length)
     const int* sel_len;      // [nsel]
     const int* sel_slot;     // [nsel] position of the chromosome in the caller's list
+    const int* sel_soff;     // [nsel] global stack: entries of the selected chromosomes before this one, per sample
     int nsel;
     int minrefbins;
     double thr;
@@ -53,7 +54,9 @@ struct SegArgs {
     int max_calls;
     int pcap;                // capacity of the per-chromosome arrays (>= longest chromosome + 1)
     unsigned* aux_g;         // when the side arrays do not fit in shared memory next to P: [blocks][pcap * aux_words] global
-    int* status;             // [0] |= 1 call overflow, 2 range-stack overflow
+    int* stack_g;            // when the stack does not fit in shared memory: per (chromosome, sample) 2 * scap ints, scap
+                             // from that chromosome's length (else in shared memory after P / aux, sized for the longest)
+    int* status;             // [0] |= 1 call overflow, 2 range-stack overflow, 4 |z| sums beyond 2^1023, 8 empty window
 };
 
 struct Best {                // lexicographic champion: value, then first occurrence (x, then y)
@@ -89,11 +92,11 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
     __shared__ double s_red[2][SEG_WARPS];
     __shared__ Best s_best[2][SEG_WARPS];
     __shared__ int s_scan[SEG_WARPS];
-    __shared__ int s_lo[SEG_STACK], s_hi[SEG_STACK];
+    __shared__ int s_cur[2];                     // the range popped by thread 0
     __shared__ int s_rows[SEG_ROWCAP];
     __shared__ int s_nrows, s_sp, s_n, s_bad, s_rnan;
     __shared__ unsigned long long s_cand[3];     // MINEFF: first passing NaN / +inf / -inf entry of a range, (x << 32) | y
-    __shared__ double s_A, s_Pm;
+    __shared__ double s_A, s_Pm, s_scale;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int sel = blockIdx.x / a.B, b = blockIdx.x % a.B;     // long chromosomes first
@@ -103,6 +106,12 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
     double* zc = a.zc + (size_t)b * a.N + cstart;                 // kept z-scores of this chromosome (global scratch)
     double* rc = MINEFF ? a.rc + (size_t)b * a.N + cstart : nullptr;
     const double* rrow = MINEFF ? a.r + (size_t)b * a.N + cstart : nullptr;
+    // pending ranges (lo, hi): disjoint and longer than min_search (triarray.py:76-82), so at most
+    // clen / (min_search + 1) + 1 are ever pending.  In shared memory after the side arrays when they fit, else a slice
+    // of global scratch sized for this chromosome.
+    const int scap = clen / (a.min_search + 1) + 1;
+    int* stk = a.stack_g ? a.stack_g + 2 * ((size_t)a.sel_soff[sel] * a.B + (size_t)b * scap)
+                         : reinterpret_cast<int*>(a.aux_g ? P + a.pcap : dh + (size_t)a.pcap * (MINEFF ? 4 : 1));
 
     // ---- 1. compaction of the kept bins (wisecondor.py:215-218: refSizes >= minrefbins) -------------------------
     if (tid == 0) { s_n = 0; s_bad = 0; s_rnan = 0; }
@@ -166,17 +175,24 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
         if (lane == 31) s_red[0][warp] = inc;
         if (lane == 0) s_red[1][warp] = la;
         __syncthreads();
-        double base = 0.0;
+        double base = 0.0, at = 0.0;
         for (int w = 0; w < warp; ++w) base += s_red[0][w];
+        for (int w = 0; w < SEG_WARPS; ++w) at += s_red[1][w];
+        // The fp32 copy is stored x 2^-k so that it never overflows (|P| <= sum |z| = at) and keeps its precision for
+        // tiny z: k = 0 unless sum |z| lies outside [2^-60, 2^100], then the scaled sum lies in [2^64, 2^65).  A power of
+        // two is exact (short of fp32 underflow, which delta covers), so the sweep, its window and the threshold test
+        // all work in scaled units; the exact phase reads the unscaled zc.
+        const int k = (at > 0x1p100 || (at > 0.0 && at < 0x1p-60)) && at < 0x1p1023 ? max(ilogb(at) - 64, -1000) : 0;
+        const double sc = ldexp(1.0, -k);
         double run = base + (inc - loc);
-        double pm = 0.0;                              // largest |prefix sum|: the scale of the fp32 rounding
+        double pm = 0.0;                              // largest |prefix sum| (scaled): the scale of the fp32 rounding
         for (int i = i0; i < i1; ++i) {
             const double v = zc[i];
-            P[i] = (float)run;
-            pm = fmax(pm, fabs(run));
+            P[i] = (float)(run * sc);
+            pm = fmax(pm, fabs(run * sc));
             if (isfinite(v)) run += v;
         }
-        if (i1 == n && i0 < n) { P[n] = (float)run; pm = fmax(pm, fabs(run)); }
+        if (i1 == n && i0 < n) { P[n] = (float)(run * sc); pm = fmax(pm, fabs(run * sc)); }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) pm = fmax(pm, __shfl_xor_sync(0xffffffffu, pm, o));
         __syncthreads();                              // s_red[0] (warp totals) has been consumed
@@ -187,18 +203,31 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
             for (int w = 0; w < SEG_WARPS; ++w) { t += s_red[1][w]; m = fmax(m, s_red[0][w]); }
             s_A = t;
             s_Pm = m;
+            s_scale = sc;
             s_sp = 1;
-            s_lo[0] = 0;
-            s_hi[0] = n;
+            stk[0] = 0;
+            stk[1] = n;
         }
         __syncthreads();
     }
-    const double A = s_A;
+    // Sums of |z| at or beyond 2^1023 can overflow double precision in numpy's sums (the reference's run values would
+    // be inf or NaN); such a chromosome is rejected as a whole (WC_ERR_ARG) instead of being located on non-finite
+    // prefix sums.  Below 2^1023 every partial sum in any order is finite.
+    if (!(s_A < 0x1p1023)) {
+        if (tid == 0) atomicOr(a.status, 4);
+        return;
+    }
+    const double scale = s_scale;                   // 2^-k of the fp32 copy; 1 unless sum |z| is outside [2^-60, 2^100]
+    const double thr_s = a.thr * scale;             // the threshold in the sweep's units (inf / 0 when out of range)
+    const double A = s_A * scale;
     // |sweep value - numpy value| <= (2 (per + 16) + 40) eps A + 3 eps |v|: prefix sums (sequential chunk of `per`, warp
     // scan, warp bases) on both ends of the run, numpy's own pairwise rounding, the reciprocal multiply.  delta = 2 x that.
     // The sweep itself runs in fp32 on an fp32 copy of the prefix sums: |fp32 score - fp64 score| <= 2^-23 Pm + 2^-21 |v|
     // (rounding of the two prefix sums, of their difference, of 1/sqrt(len) and of the product), Pm = max |prefix sum|.
-    const double delta_A = (4.0 * ((n + SEG_THREADS - 1) / SEG_THREADS) + 160.0) * SEG_EPS * A + 2.0 * 1.1920929e-07 * s_Pm;
+    // Scaled values that fall below FLT_MIN are flushed or rounded to the subnormal grid: SEG_FLT_TINY bounds that on the
+    // two prefix sums, their difference and the product.  All of delta is in the sweep's (scaled) units.
+    const double delta_A = (4.0 * ((n + SEG_THREADS - 1) / SEG_THREADS) + 160.0) * SEG_EPS * A + 2.0 * 1.1920929e-07 * s_Pm
+                           + SEG_FLT_TINY;
 
     // MINEFF: prefix counts of the ratios above c_hi / below c_lo decide the median test in O(1) for all odd lengths and
     // for even lengths unless exactly half of the run lies on the far side; then the two middle order statistics are
@@ -257,13 +286,22 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
     __shared__ int s_first[3];                      // first NaN / +inf / -inf position of the current range
 
     // ---- 3. iterative most-significant-run search (triarray.py:59-84) --------------------------------------------------
+    // the stack holds scap ranges (see stk above); status 2 is an internal assertion
+    auto push = [&](int spn, int l, int h) -> int {
+        if (spn < scap) { stk[2 * spn] = l; stk[2 * spn + 1] = h; return spn + 1; }
+        atomicOr(a.status, 2);
+        return spn;
+    };
     while (true) {
         __syncthreads();
-        const int sp = s_sp;
-        if (sp == 0) break;
-        const int lo = s_lo[sp - 1], hi = s_hi[sp - 1];
+        if (tid == 0) {
+            const int sp = s_sp;
+            if (sp > 0) { s_cur[0] = stk[2 * (sp - 1)]; s_cur[1] = stk[2 * (sp - 1) + 1]; s_sp = sp - 1; }
+            else s_cur[0] = -1;
+        }
         __syncthreads();
-        if (tid == 0) s_sp = sp - 1;
+        const int lo = s_cur[0], hi = s_cur[1];
+        if (lo < 0) break;
         const int m = hi - lo;
 
         if (MINEFF && has_bad) {
@@ -309,12 +347,8 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
                     const int slot_i = atomicAdd(&a.ncalls[b], 1);
                     if (slot_i < a.max_calls) a.calls[(size_t)b * a.max_calls + slot_i] = c; else atomicOr(a.status, 1);
                     int spn = s_sp;
-                    if ((c.y - lo) + 1 < m - a.min_search) {            // triarray.py:79
-                        if (spn < SEG_STACK) { s_lo[spn] = c.y + 1; s_hi[spn] = hi; ++spn; } else atomicOr(a.status, 2);
-                    }
-                    if (c.x - lo > a.min_search) {                      // triarray.py:76
-                        if (spn < SEG_STACK) { s_lo[spn] = lo; s_hi[spn] = c.x; ++spn; } else atomicOr(a.status, 2);
-                    }
+                    if ((c.y - lo) + 1 < m - a.min_search) spn = push(spn, c.y + 1, hi);     // triarray.py:79
+                    if (c.x - lo > a.min_search) spn = push(spn, lo, c.x);                  // triarray.py:76
                     s_sp = spn;
                 }
                 continue;
@@ -346,11 +380,7 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
                     else { c.y = fneg; c.z = -INFINITY; }
                     const int slot_i = atomicAdd(&a.ncalls[b], 1);
                     if (slot_i < a.max_calls) a.calls[(size_t)b * a.max_calls + slot_i] = c; else atomicOr(a.status, 1);
-                    if ((c.y - lo) + 1 < m - a.min_search) {            // triarray.py:79 (x == lo: never a left part)
-                        int spn = s_sp;
-                        if (spn < SEG_STACK) { s_lo[spn] = c.y + 1; s_hi[spn] = hi; ++spn; } else atomicOr(a.status, 2);
-                        s_sp = spn;
-                    }
+                    if ((c.y - lo) + 1 < m - a.min_search) s_sp = push(s_sp, c.y + 1, hi);   // triarray.py:79 (x == lo: no left part)
                 }
                 continue;
             }
@@ -417,7 +447,7 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
         // every run within delta of the true maximum M has an fp32 score >= vlow
         const double big = (double)bigf;
         const double delta = delta_A + 4.0 * 1.1920929e-07 * big;
-        if (big + delta < a.thr) continue;            // abs(champVal) < threshold for certain (triarray.py:72-73)
+        if (big + delta < thr_s) continue;            // abs(champVal) < threshold for certain (triarray.py:72-73)
         const float vlow = (float)(big - 2.0 * delta);                  // window floor on the fp32 |score|
 
         // -- diagonals that can hold the exact champion: those whose own extreme reaches the window --
@@ -463,7 +493,12 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
             }
             Best champ = cmax;                                          // triarray.py:62-70
             if (fabs(cmin.v) > champ.v) champ = cmin;
-            if (!(fabs(champ.v) < a.thr)) {                             // triarray.py:72-73
+            // Nothing in the window: with the effect-size filter every run of the range is zeroed (0 < threshold, no
+            // call); without it the window always holds the sweep's own maximum, so an empty one is an internal error.
+            // Either way no champion with x = 0x7fffffff is ever published.
+            const bool empty = cmax.x == 0x7fffffff;
+            if (empty && !MINEFF) atomicOr(a.status, 8);
+            if (!empty && !(fabs(champ.v) < a.thr)) {                   // triarray.py:72-73
                 const int slot_i = atomicAdd(&a.ncalls[b], 1);
                 if (slot_i < a.max_calls) {
                     wc_call c;
@@ -474,12 +509,8 @@ __global__ void __launch_bounds__(SEG_THREADS) wc_segment_kernel(const SegArgs a
                 }
                 int spn = s_sp;
                 const int xr = champ.x - lo, yr = champ.y - lo;        // coordinates inside the sub-triangle
-                if (yr + 1 < m - a.min_search) {                        // triarray.py:79
-                    if (spn < SEG_STACK) { s_lo[spn] = champ.y + 1; s_hi[spn] = hi; ++spn; } else atomicOr(a.status, 2);
-                }
-                if (xr > a.min_search) {                                // triarray.py:76
-                    if (spn < SEG_STACK) { s_lo[spn] = lo; s_hi[spn] = champ.x; ++spn; } else atomicOr(a.status, 2);
-                }
+                if (yr + 1 < m - a.min_search) spn = push(spn, champ.y + 1, hi);     // triarray.py:79
+                if (xr > a.min_search) spn = push(spn, lo, champ.x);                 // triarray.py:76
                 s_sp = spn;
             }
         }
@@ -534,18 +565,21 @@ extern "C" int wc_segment_batch(wc_ctx* ctx, const double* z_d, const double* r_
     std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
         return chrom_bins_h[chromosomes_h[x]] > chrom_bins_h[chromosomes_h[y]];
     });
-    std::vector<int> meta(3 * nsel);
+    std::vector<int> meta(4 * nsel);
+    long long soff = 0;                           // global stack entries per sample before each selected chromosome
     for (int i = 0; i < nsel; ++i) {
         const int c = chromosomes_h[order[i]];
         meta[i] = start[c];
         meta[nsel + i] = chrom_bins_h[c];
         meta[2 * nsel + i] = order[i];
+        meta[3 * nsel + i] = (int)soff;
+        soff += chrom_bins_h[c] / (min_search + 1) + 1;
     }
     double* zc; double* rcomp = nullptr; int* meta_d; int* status_d;
     int rc;
     if ((rc = wc_reserve(ctx, SLOT_S_ZC, (size_t)B * N * sizeof(double), (void**)&zc))) return rc;
     if (mineff && (rc = wc_reserve(ctx, SLOT_S_RC, (size_t)B * N * sizeof(double), (void**)&rcomp))) return rc;
-    if ((rc = wc_reserve(ctx, SLOT_S_META, (size_t)3 * nsel * sizeof(int), (void**)&meta_d))) return rc;
+    if ((rc = wc_reserve(ctx, SLOT_S_META, (size_t)4 * nsel * sizeof(int), (void**)&meta_d))) return rc;
     if ((rc = wc_reserve(ctx, SLOT_S_STATUS, 4 * sizeof(int), (void**)&status_d))) return rc;
     const int pcap = (maxlen + 8) & ~1;
     const size_t aux_bytes = (size_t)pcap * (sizeof(unsigned) + (mineff ? 3 * sizeof(int) : 0));
@@ -559,22 +593,36 @@ extern "C" int wc_segment_batch(wc_ctx* ctx, const double* z_d, const double* r_
         }
         if ((rc = wc_reserve(ctx, SLOT_S_AUX, (size_t)nsel * B * aux_bytes, (void**)&aux_g))) return rc;
     }
+    // pending-range stack: disjoint ranges longer than min_search.  In shared memory (sized for the longest chromosome)
+    // when that costs no resident CTA (it is touched once per range), else in a global slice per CTA sized for its own
+    // chromosome: B * sum(len / (min_search + 1) + 1) entries in all.
+    const int scap = maxlen / (min_search + 1) + 1;
+    const size_t stack_bytes = (size_t)scap * 2 * sizeof(int);
+    const void* kfn = mineff ? (const void*)wc_segment_kernel<true> : (const void*)wc_segment_kernel<false>;
+    int* stack_g = nullptr;
+    bool stack_shared = smem + stack_bytes <= 220 * 1024;
+    if (stack_shared) {
+        int without = 0, with = 0;
+        WC_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem + stack_bytes)));
+        WC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&without, kfn, SEG_THREADS, smem));
+        WC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&with, kfn, SEG_THREADS, smem + stack_bytes));
+        stack_shared = with >= without;
+    }
+    if (stack_shared) smem += stack_bytes;
+    else if ((rc = wc_reserve(ctx, SLOT_S_STACK, (size_t)soff * B * 2 * sizeof(int), (void**)&stack_g))) return rc;
     WC_CUDA(cudaEventRecord(ctx->ev[10], stream));
     WC_CUDA(cudaMemcpyAsync(meta_d, meta.data(), meta.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
     WC_CUDA(cudaMemsetAsync(status_d, 0, 4 * sizeof(int), stream));
     WC_CUDA(cudaMemsetAsync(ncalls_d, 0, (size_t)B * sizeof(int), stream));
     SegArgs a;
     a.z = z_d; a.refsz = refsizes_d; a.N = N; a.B = B; a.sel_start = meta_d; a.sel_len = meta_d + nsel;
-    a.sel_slot = meta_d + 2 * nsel; a.nsel = nsel; a.minrefbins = minrefbins; a.thr = z_threshold;
+    a.sel_slot = meta_d + 2 * nsel; a.sel_soff = meta_d + 3 * nsel; a.nsel = nsel; a.minrefbins = minrefbins; a.thr = z_threshold;
     a.min_search = min_search; a.zc = zc; a.r = r_d; a.rc = rcomp; a.c_hi = c_hi; a.c_lo = c_lo; a.cwz = cwz_d; a.cleaned = cleaned_bins_d; a.calls = calls_d;
     a.ncalls = ncalls_d; a.max_calls = max_calls; a.status = status_d; a.pcap = pcap; a.aux_g = aux_g;
-    if (mineff) {
-        WC_CUDA(cudaFuncSetAttribute(wc_segment_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        wc_segment_kernel<true><<<(unsigned)((size_t)nsel * B), SEG_THREADS, smem, stream>>>(a);
-    } else {
-        WC_CUDA(cudaFuncSetAttribute(wc_segment_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        wc_segment_kernel<false><<<(unsigned)((size_t)nsel * B), SEG_THREADS, smem, stream>>>(a);
-    }
+    a.stack_g = stack_g;
+    WC_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (mineff) wc_segment_kernel<true><<<(unsigned)((size_t)nsel * B), SEG_THREADS, smem, stream>>>(a);
+    else wc_segment_kernel<false><<<(unsigned)((size_t)nsel * B), SEG_THREADS, smem, stream>>>(a);
     WC_CUDA(cudaGetLastError());
     WC_CUDA(cudaEventRecord(ctx->ev[11], stream));
     int status = 0;
@@ -582,7 +630,13 @@ extern "C" int wc_segment_batch(wc_ctx* ctx, const double* z_d, const double* r_
     WC_CUDA(cudaStreamSynchronize(stream));       // meta/status host buffers; the call is documented as synchronous
     ctx->timed_mask |= 1u << 5;
     ctx->counter[6] = 1;
-    if (status & 2) { wc_set_error("segmentation: more than %d pending ranges on one chromosome", SEG_STACK); return WC_ERR_INTERNAL; }
+    if (status & 2) { wc_set_error("segmentation: pending ranges overflowed the range stack (internal error)"); return WC_ERR_INTERNAL; }
+    if (status & 8) { wc_set_error("segmentation: the error window of a range selected no run"); return WC_ERR_INTERNAL; }
+    if (status & 4) {
+        wc_set_error("segmentation: the sum of |z| over a chromosome is at least 2^1023 (8.99e307); its run sums could "
+                     "overflow double precision");
+        return WC_ERR_ARG;
+    }
     if (status & 1) { wc_set_error("segmentation: more than max_calls=%d calls for one sample", max_calls); return WC_ERR_ARG; }
     return WC_OK;
 }
