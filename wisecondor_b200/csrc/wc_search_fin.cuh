@@ -308,13 +308,16 @@ __global__ void __launch_bounds__(SELH_WARPS * 32, 5) wc_fin_select_hist_kernel(
     // ---- pass 1: histogram of the live filter distances ----
     // bucket scale: distances in [d0, dmax] = [0, the row's final threshold].  A row nobody published a threshold for still
     // carries the initial one (1e10 or 3e38, or ~0 without a table): one more pass for the smallest and largest entry
-    // below 1e10 (entries from there on - fillers, inf, NaN - rank last and are dropped at the end, wisetools.py:312-314).
+    // that can be below 1e10 (entries from there on - fillers, inf, NaN - rank last and are dropped at the end,
+    // wisetools.py:312-314).  The test is on the filter distance, so it takes the filter's margin: an exact distance just
+    // below 1e10 may be filtered a few ulps above it.
     double d0 = 0.0, dmax = dist_of_key(tfinal);
     if (!(dmax < 1e10)) {
+        const double cut = 1e10 + a.mcoef * (a.norms[row] + 1e10) + madd_of(a);
         double mn = INFINITY, mx = -INFINITY;
         sweep([&](u64 key, int, bool valid) {
             const double d = dist_of_key(key);
-            if (valid && key <= tfinal && d < 1e10) { mn = fmin(mn, d); mx = fmax(mx, d); }
+            if (valid && key <= tfinal && d <= cut) { mn = fmin(mn, d); mx = fmax(mx, d); }
         });
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
