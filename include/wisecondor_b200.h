@@ -195,7 +195,9 @@ int wc_pca_apply(wc_ctx* ctx, const double* masked_d, int N, int S, const double
  *   count_d  DEVICE N int32
  *   rev_off_d DEVICE N+1 int32, rev_idx_d DEVICE N x wc_table_stride(k) int32: the reverse table (CSR) - for every bin
  *            the bins that use it as a reference bin; lets the later passes of wc_zscore_batch touch only what a
- *            newly marked bin can change */
+ *            newly marked bin can change
+ * k (the npz's refsize) may be any value >= 1 with N x wc_table_stride(k) < 2^31 (k <= 37 260 at 50 kb, 7 452 at
+ * 10 kb); larger values are refused with WC_ERR_ARG before any memory is touched. */
 int wc_table_stride(int k);
 int wc_test_table(wc_ctx* ctx, const int32_t* indexes_d, const double* distances_d, int N, int k,
                   const int* chrom_bins_h, int nchrom, double cutoff, int32_t* table_d, int32_t* count_d,
@@ -221,7 +223,9 @@ int wc_apply_pca(wc_ctx* ctx, const double* x_d, int B, int N, const double* pca
  *   z_d, r_d DEVICE B x N float64 (sample-major), refsizes_d DEVICE B x N int32: resultsZ, resultsR, refSizes of
  *   the last pass;  asdef_d DEVICE B float64: stdDevSum / stdDevNum.  Bit-identical to the reference (numpy's
  *   summation order).  copy_init_d (DEVICE N x ldb, or NULL = test_d) is trySample's `testCopy`: the values the
- *   reference bins are gathered from in the first pass, -1 where already marked.  Asynchronous. */
+ *   reference bins are gathered from in the first pass, -1 where already marked.  k: the table's refsize, as given
+ *   to wc_test_table (any k >= 1 with N x wc_table_stride(k) < 2^31; above 512 the wide-refsize kernels run).
+ *   Asynchronous. */
 int wc_zscore_batch(wc_ctx* ctx, const double* test_d, const double* copy_init_d, int N, int B, int ldb,
                     const int32_t* table_d, const int32_t* count_d, const int32_t* rev_off_d, const int32_t* rev_idx_d,
                     int k, double z_threshold, int repeats, double* z_d, double* r_d, int32_t* refsizes_d,

@@ -72,3 +72,59 @@ __device__ __forceinline__ double np_sum_thread(F f, int n) {
     }
     return ret;
 }
+
+// The same order, fed one element at a time: begin(n) fixes the split tree of n elements, push() takes them in index
+// order, and after the n-th push `res` holds the sum.  The caller needs no storage for the elements, so it can drop
+// values on the fly (numpy sums the compacted array: the tree is that of the kept count).  The stack holds, per
+// ancestor of the current leaf, either the pending right half's length or the finished left half's sum; it is touched
+// once per leaf (>= 64 elements).  The leaf's eight accumulators form a ring that rotates by one per element, so
+// r0 always receives element p, without run-time register indexing; `full` is a multiple of 8, so the ring is back in
+// place when the accumulators are combined.
+constexpr int NP_STREAM_DEPTH = 26;    // n <= 128 * 2^24 as above
+struct NpStream {
+    double r0, r1, r2, r3, r4, r5, r6, r7, res;
+    int leaf, p, full, d;                      // current leaf's length, position in it, 8-multiple part; frames
+    int rlen[NP_STREAM_DEPTH];                 // > 0: left half in progress, right half of this length pending
+    double lsum[NP_STREAM_DEPTH];              // right half in progress: the left half's sum
+
+    __device__ __forceinline__ void descend(int len) {       // start the leftmost leaf of a piece of len elements
+        while (len > 128) {
+            int h = len / 2;
+            h -= h & 7;
+            rlen[d] = len - h;
+            ++d;
+            len = h;
+        }
+        leaf = len; p = 0; full = len - (len & 7); res = 0.0;
+    }
+    __device__ __forceinline__ void begin(int n) { d = 0; descend(n); }    // n == 0: res = 0.0 at once
+
+    __device__ __forceinline__ void push(double v) {
+        if (p < full) {
+            const double t = p < 8 ? v : __dadd_rn(r0, v);
+            r0 = r1; r1 = r2; r2 = r3; r3 = r4; r4 = r5; r5 = r6; r6 = r7; r7 = t;
+            if (p + 1 == full)
+                res = __dadd_rn(__dadd_rn(__dadd_rn(r0, r1), __dadd_rn(r2, r3)), __dadd_rn(__dadd_rn(r4, r5), __dadd_rn(r6, r7)));
+        } else {
+            res = __dadd_rn(res, v);                              // n < 8, or the n % 8 tail
+        }
+        if (++p == leaf) finish_leaf();
+    }
+    __device__ __forceinline__ void finish_leaf() {
+        double s = res;
+        while (d > 0) {
+            const int f = d - 1;
+            if (rlen[f] > 0) {                                    // a left half is done: start its right sibling
+                lsum[f] = s;
+                const int len = rlen[f];
+                rlen[f] = 0;
+                descend(len);
+                return;
+            }
+            s = __dadd_rn(lsum[f], s);                            // a right half is done: (left + right) goes up
+            d = f;
+        }
+        res = s;
+        leaf = -1;                                                // finished: further pushes are a caller error
+    }
+};

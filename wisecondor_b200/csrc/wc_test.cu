@@ -416,6 +416,90 @@ __global__ void __launch_bounds__(ZS_WARPS * 32) wc_zscore_pairs_kernel(const ZA
     }
 }
 
+// ---- K8w: the same passes for k > 512 ---------------------------------------------------------------------------
+// K8's fast path unrolls numpy's split tree to three levels and its slow path keeps k doubles per warp in shared memory,
+// which bounds it at 512.  Here every lane evaluates the split tree over its own kept values in one streaming walk
+// (NpStream), so the cost per value is constant and nothing is staged.  The layout is K8's: in the full kernel a warp
+// is 32 samples x one bin, the lanes walk the bin's table row in lockstep (a broadcast index load, one coalesced 256 B
+// gather per reference bin) and differ only in which values they push.  The tree must be that of the kept count,
+// which is only known after a walk: the first walk assumes nothing is dropped (tree of `count`); a lane that dropped
+// something walks again with the tree of its kept count.  Then one more walk for sum((x - mean)^2).
+template <bool DEV>
+__device__ __forceinline__ double zw_walk(const double* cp, const int* tab, int cnt, size_t ldb, int n_tree, double mean,
+                                          int& kept) {
+    NpStream acc;
+    acc.begin(n_tree);
+    int nk = 0;
+    auto feed = [&](double v) {
+        if (v >= 0.0) {                                   // refData[refData >= 0] (wisetools.py:425): NaN never passes
+            ++nk;
+            if (DEV) {
+                const double d = __dsub_rn(v, mean);
+                v = __dmul_rn(d, d);
+            }
+            acc.push(v);
+        }
+    };
+    int m = 0;
+    for (; m + 8 <= cnt; m += 8) {
+        const int4 i0 = *reinterpret_cast<const int4*>(tab + m), i1 = *reinterpret_cast<const int4*>(tab + m + 4);
+        double v[8];
+        v[0] = cp[(size_t)i0.x * ldb]; v[1] = cp[(size_t)i0.y * ldb]; v[2] = cp[(size_t)i0.z * ldb]; v[3] = cp[(size_t)i0.w * ldb];
+        v[4] = cp[(size_t)i1.x * ldb]; v[5] = cp[(size_t)i1.y * ldb]; v[6] = cp[(size_t)i1.z * ldb]; v[7] = cp[(size_t)i1.w * ldb];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) feed(v[j]);
+    }
+    for (; m < cnt; ++m) feed(cp[(size_t)tab[m] * ldb]);
+    kept = nk;
+    return acc.res;                                       // numpy's sum iff nk == n_tree
+}
+
+__device__ __forceinline__ ZsSlow zw_lane(const double* cp, const int* tab, int cnt, size_t ldb) {
+    ZsSlow o;
+    double sum;
+    int n_tree = cnt;
+    for (;;) {                                            // at most twice: the second walk uses the kept count
+        sum = zw_walk<false>(cp, tab, cnt, ldb, n_tree, 0.0, o.n);
+        if (o.n == n_tree) break;
+        n_tree = o.n;
+    }
+    o.mean = __ddiv_rn(sum, (double)o.n);                                                       // np_mean (:426)
+    int unused;
+    o.sd = sqrt(__ddiv_rn(zw_walk<true>(cp, tab, cnt, ldb, o.n, o.mean, unused), (double)o.n));   // np_std (:427)
+    return o;
+}
+
+__device__ __forceinline__ void zw_store(const ZArgs& a, int i, int s, const ZsSlow& o) {
+    const size_t idx = (size_t)i * a.ldb + s;
+    const double x = a.test[idx];
+    a.z[idx] = __ddiv_rn(__dsub_rn(x, o.mean), o.sd);                                          // wisetools.py:431
+    a.r[idx] = __ddiv_rn(x, o.mean);                                                           // wisetools.py:432
+    a.refsz[idx] = o.n;
+    a.sd[idx] = o.sd;
+}
+
+__global__ void __launch_bounds__(ZS_WARPS * 32) wc_zscore_wide_kernel(const ZArgs a) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int nwarps = blockDim.x >> 5;
+    if (a.npairs != nullptr && *a.npairs <= a.pair_limit) return;       // the pair kernel handles this pass
+    const int s = blockIdx.y * 32 + lane;                // < ldb by construction
+    const int bin_end = min(a.N, (int)(blockIdx.x + 1) * ZS_BINS_PER_CTA);
+    for (int i = blockIdx.x * ZS_BINS_PER_CTA + warp; i < bin_end; i += nwarps)
+        zw_store(a, i, s, zw_lane(a.copy + s, a.table + (size_t)i * a.k, a.count[i], (size_t)a.ldb));
+}
+
+// Dirty-pair pass for k > 512: one listed pair per thread, the same walk as the full kernel.
+__global__ void __launch_bounds__(ZS_WARPS * 32) wc_zscore_wide_pairs_kernel(const ZArgs a, const int* __restrict__ pairs,
+                                                                             const int* __restrict__ npairs) {
+    const int n_pairs = *npairs;
+    if (n_pairs > a.pair_limit) return;                   // too many for scattered gathers: the full kernel runs instead
+    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n_pairs; e += gridDim.x * blockDim.x) {
+        const int code = pairs[e];
+        const int i = code / a.ldb, s = code - i * a.ldb;
+        zw_store(a, i, s, zw_lane(a.copy + s, a.table + (size_t)i * a.k, a.count[i], (size_t)a.ldb));
+    }
+}
+
 // stdDevSum / stdDevNum accumulated bin by bin like the reference's Python loop (wisetools.py:428-430, 435): a strictly
 // sequential sum per sample, so the parallelism is across samples only.  A CTA owns 32 samples: all eight warps stream
 // the [64 bins][32 samples] tiles of the sigma array into shared memory (coalesced, cp.async, double buffered) and warp 0
@@ -500,6 +584,18 @@ int upload_row_ranges(wc_ctx* ctx, int N, const int* chrom_bins_h, int nchrom, i
 
 extern "C" int wc_table_stride(int k) { return (k + 3) & ~3; }
 
+// The table, the reverse table and the dirty-pair codes are indexed with int32: N x wc_table_stride(k) must stay below
+// 2^31 (k <= 37 260 at 50 kb, N = 57 633; k <= 7 452 at 10 kb).  Checked before any memory is touched.
+static int check_table_size(int N, int k) {
+    const long long stride = ((long long)k + 3) & ~3LL;
+    if ((long long)N * stride >= (1LL << 31)) {
+        wc_set_error("bad argument: N x wc_table_stride(k) = %d x %lld must be below 2^31 (refsize too large for %d bins)",
+                     N, stride, N);
+        return WC_ERR_ARG;
+    }
+    return WC_OK;
+}
+
 extern "C" int wc_test_table(wc_ctx* ctx, const int32_t* indexes_d, const double* distances_d, int N, int k,
                              const int* chrom_bins_h, int nchrom, double cutoff, int32_t* table_d, int32_t* count_d,
                              int32_t* rev_off_d, int32_t* rev_idx_d, void* stream_v) {
@@ -509,10 +605,11 @@ extern "C" int wc_test_table(wc_ctx* ctx, const int32_t* indexes_d, const double
     long long tot = 0;
     for (int c = 0; c < nchrom; ++c) { WC_CHECK_ARG(chrom_bins_h[c] >= 0); tot += chrom_bins_h[c]; }
     WC_CHECK_ARG(tot == N);
+    int rc;
+    if ((rc = check_table_size(N, k))) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
     WC_CUDA(cudaSetDevice(ctx->device));
     int* cs_d; int* ce_d;
-    int rc;
     if ((rc = upload_row_ranges(ctx, N, chrom_bins_h, nchrom, SLOT_ROWCS, SLOT_ROWCE, &cs_d, &ce_d, stream))) return rc;
     const int blocks = (int)(((size_t)N * 32 + 255) / 256);
     const int ldk = wc_table_stride(k);
@@ -578,14 +675,15 @@ extern "C" int wc_zscore_batch(wc_ctx* ctx, const double* test_d, const double* 
                                int32_t* refsizes_d, double* asdef_d, void* stream_v) {
     WC_CHECK_ARG(ctx != nullptr && test_d != nullptr && table_d != nullptr && count_d != nullptr);
     WC_CHECK_ARG(z_d != nullptr && r_d != nullptr && refsizes_d != nullptr && asdef_d != nullptr);
-    WC_CHECK_ARG(N > 0 && B > 0 && ldb >= B && ldb % 32 == 0 && k >= 1 && k <= 512 && repeats >= 1);
+    WC_CHECK_ARG(N > 0 && B > 0 && ldb >= B && ldb % 32 == 0 && k >= 1 && repeats >= 1);
     WC_CHECK_ARG(repeats == 1 || (rev_off_d != nullptr && rev_idx_d != nullptr));
     WC_CHECK_ARG((size_t)N * ldb < ((size_t)1 << 31));
+    int rc;
+    if ((rc = check_table_size(N, k))) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
     WC_CUDA(cudaSetDevice(ctx->device));
     const size_t elems = (size_t)N * ldb;
     double* copy; double* zt; double* rt; int* nt; double* sd; unsigned char* dirty; int* pairs; int* npairs;
-    int rc;
     if ((rc = wc_reserve(ctx, SLOT_T_COPY, elems * sizeof(double), (void**)&copy))) return rc;
     if ((rc = wc_reserve(ctx, SLOT_T_ZT, elems * sizeof(double), (void**)&zt))) return rc;
     if ((rc = wc_reserve(ctx, SLOT_T_RT, elems * sizeof(double), (void**)&rt))) return rc;
@@ -597,9 +695,12 @@ extern "C" int wc_zscore_batch(wc_ctx* ctx, const double* test_d, const double* 
                             stream));                                                                   // wisetools.py:442
     const int warps = ZS_WARPS;
     const int ldk = wc_table_stride(k);
-    const size_t smem = (size_t)warps * ldk * sizeof(double);     // slow-path scratch only
-    WC_CUDA(cudaFuncSetAttribute(wc_zscore_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    WC_CUDA(cudaFuncSetAttribute(wc_zscore_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const bool wide = k > 512;                  // K8's sums and slow-path scratch stop at 512 values: K8w beyond
+    const size_t smem = wide ? 0 : (size_t)warps * ldk * sizeof(double);     // slow-path scratch only
+    if (!wide) {
+        WC_CUDA(cudaFuncSetAttribute(wc_zscore_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        WC_CUDA(cudaFuncSetAttribute(wc_zscore_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    }
     ZArgs a;
     a.test = test_d; a.copy = copy; a.table = table_d; a.count = count_d; a.N = N; a.B = B; a.ldb = ldb; a.k = ldk;
     a.z = zt; a.r = rt; a.refsz = nt; a.sd = sd; a.npairs = nullptr;
@@ -608,7 +709,8 @@ extern "C" int wc_zscore_batch(wc_ctx* ctx, const double* test_d, const double* 
     a.pair_limit = (int)std::min<size_t>((size_t)N * B / 8, (size_t)0x7fffffff);
     long long launches = 0;
     const dim3 zgrid((N + ZS_BINS_PER_CTA - 1) / ZS_BINS_PER_CTA, ldb / 32);
-    wc_zscore_kernel<<<zgrid, warps * 32, smem, stream>>>(a);       // first pass: every (bin, sample) pair
+    if (wide) wc_zscore_wide_kernel<<<zgrid, warps * 32, 0, stream>>>(a);
+    else wc_zscore_kernel<<<zgrid, warps * 32, smem, stream>>>(a);       // first pass: every (bin, sample) pair
     ++launches;
     if (repeats > 1) {
         if ((rc = wc_reserve(ctx, SLOT_T_DIRTY, elems, (void**)&dirty))) return rc;
@@ -620,8 +722,13 @@ extern "C" int wc_zscore_batch(wc_ctx* ctx, const double* test_d, const double* 
             wc_mark_kernel<<<eblocks, 256, 0, stream>>>(zt, copy, N, B, ldb, z_threshold, rev_off_d, rev_idx_d, dirty);
             wc_compact_kernel<<<eblocks, 256, 0, stream>>>(dirty, elems, pairs, npairs + rep);
             a.npairs = npairs + rep;                   // exactly one of the next two kernels does the pass
-            wc_zscore_pairs_kernel<<<4 * ctx->sm_count, warps * 32, smem, stream>>>(a, pairs, npairs + rep);
-            wc_zscore_kernel<<<zgrid, warps * 32, smem, stream>>>(a);
+            if (wide) {
+                wc_zscore_wide_pairs_kernel<<<4 * ctx->sm_count, warps * 32, 0, stream>>>(a, pairs, npairs + rep);
+                wc_zscore_wide_kernel<<<zgrid, warps * 32, 0, stream>>>(a);
+            } else {
+                wc_zscore_pairs_kernel<<<4 * ctx->sm_count, warps * 32, smem, stream>>>(a, pairs, npairs + rep);
+                wc_zscore_kernel<<<zgrid, warps * 32, smem, stream>>>(a);
+            }
             launches += 4;
         }
     }

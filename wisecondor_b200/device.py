@@ -139,16 +139,22 @@ def pad32(b):
 
 class ReferenceTable(object):
     """Device-resident form of a reference npz for the test path: per bin the global ids of its usable reference
-    bins (`index[distances < cutoff]` mapped out of other-chromosome coordinates, wisetools.py:420-424)."""
+    bins (`index[distances < cutoff]` mapped out of other-chromosome coordinates, wisetools.py:420-424).  Any refsize
+    with N x wc_table_stride(refsize) < 2^31 is accepted; the table and the reverse table take 2 x N x stride x 4 B
+    of device memory (1.9 GB at 50 kb with refsize 4096)."""
 
     def __init__(self, indexes, distances, masked_sizes, cutoff, device=0):
         self.masked_sizes = [int(v) for v in masked_sizes]
         self.n, self.k = int(indexes.shape[0]), int(indexes.shape[1])
+        stride = _cabi.lib().wc_table_stride(self.k)
+        if self.n * stride >= 2 ** 31:
+            raise _cabi.WisecondorError("reference table of %d bins x refsize %d (row stride %d) needs N x stride < 2^31"
+                                        % (self.n, self.k, stride))
         self.cutoff = float(cutoff)
         idx = _mem.to_device(np.ascontiguousarray(indexes, dtype=np.int32), device)
         dst = _mem.to_device(np.ascontiguousarray(distances, dtype=np.float64), device)
         self.device = idx.device
-        self.table = _mem.empty((self.n, _cabi.lib().wc_table_stride(self.k)), I32, like=idx)
+        self.table = _mem.empty((self.n, stride), I32, like=idx)
         self.count = _mem.empty((self.n,), I32, like=idx)
         # reverse table (CSR): which bins use bin j as a reference bin
         self.rev_off = _mem.empty((self.n + 1,), I32, like=idx)
