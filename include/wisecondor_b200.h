@@ -112,7 +112,7 @@ int wc_debug_filter_scores(wc_ctx* ctx, float* out_d, int ld);
 int wc_debug_pivot_select(wc_ctx* ctx, const float* n32_d, int N, int R, int* ids_d);
 
 /* ABI version of this header; wc_abi_version() returns the one the library was built from (the binding refuses a mismatch). */
-#define WC_ABI_VERSION 2
+#define WC_ABI_VERSION 3
 int wc_abi_version(void);
 
 /* ---- newref: reference-bin search --------------------------------------------------------------------- */
@@ -121,7 +121,7 @@ int wc_abi_version(void);
  *   corrected_d  DEVICE  N x S float64, bin-major C order (row = bin, S contiguous): the `correctedData` of
  *                        the prep npz (wisecondor.py:106)
  *   chrom_bins_h HOST    nchrom masked bins per chromosome (`maskedChromBins`, wisecondor.py:93); sum == N
- *   refsize              `selectRefAmount` / -refsize (wisecondor.py:379), 1..384
+ *   refsize              `selectRefAmount` / -refsize (wisecondor.py:379), 1..384 (larger: wc_newref_topk_wide)
  *   idx_d        DEVICE  (row_end-row_begin) x refsize int32: positions in the other-chromosome concatenation
  *   dist_d       DEVICE  (row_end-row_begin) x refsize float64: squared distances, ascending
  * Rows are the first `refsize` candidates ordered by (distance, index); unfilled slots hold -1 / 1e10.
@@ -129,6 +129,17 @@ int wc_abi_version(void);
  * subtract/multiply/add) and are bit-identical to the reference's.  Synchronous. */
 int wc_newref_topk(wc_ctx* ctx, const double* corrected_d, int N, int S, const int* chrom_bins_h, int nchrom,
                    int row_begin, int row_end, int refsize, int32_t* idx_d, double* dist_d, void* stream);
+
+/* Largest refsize wc_newref_topk_wide accepts. */
+#define WC_WIDE_REFSIZE_MAX 4096
+
+/* The same search for 1 <= refsize <= WC_WIDE_REFSIZE_MAX, with the arguments and output contract of wc_newref_topk
+ * (larger refsize: WC_ERR_ARG before any memory is touched).  Computes every distance of a chunk of target rows exactly,
+ * in the reference's operation order, then selects and ranks each row; chunks of a multiple of 128 rows whose distances
+ * take at most 1 GiB of device memory.  Phases: 1 = distances, 2 = select + rank; counter 0 = kernel launches,
+ * 2 = rows per chunk.  Synchronous. */
+int wc_newref_topk_wide(wc_ctx* ctx, const double* corrected_d, int N, int S, const int* chrom_bins_h, int nchrom,
+                        int row_begin, int row_end, int refsize, int32_t* idx_d, double* dist_d, void* stream);
 
 /* Same call with HOST buffers (copies in and out inside the call): the form toolNewrefPart
  * (wisecondor.py:111-132) would bind. */

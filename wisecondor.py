@@ -451,11 +451,11 @@ def buildParser():
     sub = parser.add_subparsers()
 
     def refsize(text):
-        """-refsize: the reference accepts any positive count (wisecondor.py:379); the device search keeps a bin's candidates
-        in buffers sized for at most 384 of them, so larger values are refused HERE, before any work is done."""
+        """-refsize: the reference accepts any positive count (wisecondor.py:379); the device search takes up to 4096
+        (the wide-refsize search above 384), so larger values are refused HERE, before any work is done."""
         value = int(text)
-        if not 1 <= value <= 384:
-            raise argparse.ArgumentTypeError("refsize must be between 1 and 384 on the B200 search (got %d)" % value)
+        if not 1 <= value <= 4096:
+            raise argparse.ArgumentTypeError("refsize must be between 1 and 4096 on the B200 search (got %d)" % value)
         return value
 
     p = sub.add_parser('convert', description='Convert and filter a bam file to an npz')
@@ -469,7 +469,7 @@ def buildParser():
     p = sub.add_parser('newref', description='Create a new reference using healthy reference samples')
     p.add_argument('infiles', type=str, nargs='*', help='Reference sample npz files')
     p.add_argument('outfile', type=str, help='Reference output npz')
-    p.add_argument('-refsize', type=refsize, default=100, help='Amount of reference locations per target (1..384)')
+    p.add_argument('-refsize', type=refsize, default=100, help='Amount of reference locations per target (1..4096)')
     p.add_argument('-binsize', type=int, default=None, help='Scale samples to this binsize (multiples only)')
     p.add_argument('-cpus', type=int, default=1, help='Kept for compatibility: raises the number of parts')
     p.add_argument('-parts', type=int, default=1, help='Split reference finding in this many row parts')

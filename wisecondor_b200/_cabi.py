@@ -9,11 +9,11 @@ import os
 from . import build as _build
 
 _LIB = None
-ABI_VERSION = 2      # include/wisecondor_b200.h: WC_ABI_VERSION
+ABI_VERSION = 3      # include/wisecondor_b200.h: WC_ABI_VERSION
 
 SYMBOLS = [
     "wc_create", "wc_destroy", "wc_last_error", "wc_version", "wc_abi_version", "wc_debug_filter_scores", "wc_debug_pivot_select", "wc_sm_count", "wc_last_phase_ms",
-    "wc_last_counter", "wc_device_count", "wc_dev_alloc", "wc_dev_free", "wc_copy_h2d", "wc_copy_d2h", "wc_dev_sync", "wc_newref_topk", "wc_newref_topk_host",
+    "wc_last_counter", "wc_device_count", "wc_dev_alloc", "wc_dev_free", "wc_copy_h2d", "wc_copy_d2h", "wc_dev_sync", "wc_newref_topk", "wc_newref_topk_wide", "wc_newref_topk_host",
     "wc_newref_shard_dims", "wc_newref_shard_begin", "wc_newref_shard_sweep", "wc_newref_shard_finish", "wc_debug_sym_plan", "wc_debug_profile", "wc_set_option",
     "wc_newref_mask", "wc_newref_normalize", "wc_pca_gram", "wc_pca_apply",
     "wc_table_stride", "wc_test_table", "wc_test_prep", "wc_apply_pca", "wc_zscore_batch", "wc_segment_batch",
@@ -74,6 +74,8 @@ def lib():
     L.wc_dev_sync.argtypes = [vp]
     L.wc_newref_topk.restype = ci
     L.wc_newref_topk.argtypes = [vp, vp, ci, ci, vp, ci, ci, ci, ci, vp, vp, vp]
+    L.wc_newref_topk_wide.restype = ci
+    L.wc_newref_topk_wide.argtypes = [vp, vp, ci, ci, vp, ci, ci, ci, ci, vp, vp, vp]
     L.wc_newref_topk_host.restype = ci
     L.wc_newref_topk_host.argtypes = [vp, vp, ci, ci, vp, ci, ci, ci, ci, vp, vp]
     L.wc_newref_shard_dims.restype = ci

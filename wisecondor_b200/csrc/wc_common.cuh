@@ -50,7 +50,8 @@ enum {
     SLOT_T_REVCNT = 44, SLOT_T_REVCUR, SLOT_T_DIRTY, SLOT_T_PAIRS,
     SLOT_S_ZC = 32, SLOT_S_META, SLOT_S_STATUS, SLOT_S_RC, SLOT_S_AUX,                                                       // segmentation
     SLOT_P_FIRST = 40,                                                                                 // newref prep
-    SLOT_FIN_J = 48, SLOT_FIN_D, SLOT_FIN_P, SLOT_FIN_GRP                                              // K6 split form: shortlists, exact distances, work list
+    SLOT_FIN_J = 48, SLOT_FIN_D, SLOT_FIN_P, SLOT_FIN_GRP,                                             // K6 split form: shortlists, exact distances, work list
+    SLOT_WIDE_D = 52, SLOT_WIDE_ROWS                                                                   // wide-refsize search: chunk distances, exclusion ranges
 };
 
 // State of a sharded symmetric search between its three calls (wc_newref_shard_begin / _sweep / _finish).

@@ -1133,6 +1133,7 @@ namespace {
 // and the live A panels (grid/G of them) stay L2-resident.  Row blocks left after the last full round are cut into
 // contiguous ranges that level the CTAs' tile counts (water-filling), so the balance of the plain equal split is kept.
 #include "wc_search_fin.cuh"      // K6 split form: streaming re-score + rank, and the K6 launch shared by both search entries
+#include "wc_search_wide.cuh"     // K5w / K6w: the wide-refsize search (wc_newref_topk_wide)
 
 struct Piece { int cta, rb, q0, q1, step, seg, pass; };
 void schedule_pieces(const std::vector<int>& prefix, int nrb, int grid, int G, bool rounds_on, int pass,
@@ -1940,6 +1941,82 @@ extern "C" int wc_newref_topk_host(wc_ctx* ctx, const double* corrected_h, int N
         WC_CUDA(cudaStreamSynchronize(0));
         WC_CUDA(cudaStreamSynchronize(ctx->d2h_stream));
     }
+    return WC_OK;
+}
+
+extern "C" int wc_newref_topk_wide(wc_ctx* ctx, const double* corrected_d, int N, int S, const int* chrom_bins_h,
+                                   int nchrom, int row_begin, int row_end, int refsize, int32_t* idx_d, double* dist_d,
+                                   void* stream_v) {
+    WC_CHECK_ARG(ctx != nullptr);
+    WC_CHECK_ARG(corrected_d != nullptr && chrom_bins_h != nullptr);
+    WC_CHECK_ARG(N > 0 && S > 0 && nchrom > 0);
+    WC_CHECK_ARG(refsize >= 1 && refsize <= WC_WIDE_REFSIZE_MAX);
+    WC_CHECK_ARG(row_begin >= 0 && row_begin <= row_end && row_end <= N);
+    long long tot = 0;
+    for (int c = 0; c < nchrom; ++c) {
+        WC_CHECK_ARG(chrom_bins_h[c] >= 0);
+        tot += chrom_bins_h[c];
+    }
+    WC_CHECK_ARG(tot == N);
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+    WC_CUDA(cudaSetDevice(ctx->device));
+    for (int i = 0; i < 4; ++i) ctx->phase_ms[i] = 0.0;
+    for (int i = 0; i < 5; ++i) ctx->counter[i] = 0;
+    ctx->timed_mask &= ~0xfu;
+    const int rows = row_end - row_begin;
+    if (rows == 0) return WC_OK;
+    WC_CHECK_ARG(idx_d != nullptr && dist_d != nullptr);
+
+    // exclusion range [cs, ce) of every bin: its own chromosome
+    std::vector<int> rc_h(2 * (size_t)N);
+    for (int c = 0, pos = 0; c < nchrom; pos += chrom_bins_h[c++])
+        for (int i = 0; i < chrom_bins_h[c]; ++i) { rc_h[pos + i] = pos; rc_h[(size_t)N + pos + i] = pos + chrom_bins_h[c]; }
+    // rows per chunk: a multiple of 128 whose distances fit WIDE_CHUNK_BYTES (at least 128)
+    const size_t row_bytes = (size_t)N * sizeof(double);
+    int R = (int)std::min<size_t>(WIDE_CHUNK_BYTES / row_bytes / 128 * 128, (size_t)(rows + 127) / 128 * 128);
+    if (R < 128) R = 128;
+    int* rc_d;
+    double* D;
+    int rc;
+    if ((rc = wc_reserve(ctx, SLOT_WIDE_ROWS, rc_h.size() * sizeof(int), (void**)&rc_d))) return rc;
+    if ((rc = wc_reserve(ctx, SLOT_WIDE_D, (size_t)R * row_bytes, (void**)&D))) return rc;
+    WC_CUDA(cudaMemcpyAsync(rc_d, rc_h.data(), rc_h.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
+    int P = 32;
+    while (P < refsize) P <<= 1;
+    const size_t smem = (size_t)P * (sizeof(u64) + sizeof(int));
+    WC_CUDA(cudaFuncSetAttribute(wc_wide_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+
+    WideRankArgs ra;
+    ra.D = D;
+    ra.N = N;
+    ra.k = refsize;
+    ra.row_cs = rc_d;
+    ra.row_ce = rc_d + N;
+    double ms_dist = 0.0, ms_rank = 0.0;
+    long long launches = 0;
+    for (int c0 = row_begin; c0 < row_end; c0 += R) {
+        const int r = std::min(R, row_end - c0);
+        WC_CUDA(cudaEventRecord(ctx->ev[0], stream));
+        const dim3 grid((N + WIDE_TILE - 1) / WIDE_TILE, (r + WIDE_TILE - 1) / WIDE_TILE);
+        wc_wide_dist_kernel<<<grid, WIDE_DIST_THREADS, 0, stream>>>(corrected_d, N, S, c0, r, rc_d, rc_d + N, D);
+        WC_CUDA(cudaGetLastError());
+        WC_CUDA(cudaEventRecord(ctx->ev[1], stream));
+        ra.row0 = c0;
+        ra.idx_out = idx_d + (size_t)(c0 - row_begin) * refsize;
+        ra.dist_out = dist_d + (size_t)(c0 - row_begin) * refsize;
+        wc_wide_rank_kernel<<<r, WIDE_RANK_THREADS, smem, stream>>>(ra);
+        WC_CUDA(cudaGetLastError());
+        WC_CUDA(cudaEventRecord(ctx->ev[2], stream));
+        WC_CUDA(cudaEventSynchronize(ctx->ev[2]));        // per-chunk phase times (the call is synchronous anyway)
+        float ms = 0.f;
+        WC_CUDA(cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1])); ms_dist += ms;
+        WC_CUDA(cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2])); ms_rank += ms;
+        launches += 2;
+    }
+    ctx->phase_ms[1] = ms_dist;
+    ctx->phase_ms[2] = ms_rank;
+    ctx->counter[0] = launches;
+    ctx->counter[2] = R;
     return WC_OK;
 }
 

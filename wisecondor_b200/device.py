@@ -14,12 +14,11 @@ from ._mem import ptr as _ptr, stream_ptr as _stream_ptr, require as _require_cu
 F64, I32, U8 = np.float64, np.int32, np.uint8
 
 
-def newref_topk(corrected, chrom_bins, row_begin, row_end, refsize, out_idx=None, out_dist=None):
-    """Reference-bin search for target rows [row_begin, row_end) (wisetools.py:364-398, 298-325).
+NARROW_REFSIZE_MAX = 384     # wc_newref_topk (and the sharded symmetric search)
+WIDE_REFSIZE_MAX = 4096      # wc_newref_topk_wide: include/wisecondor_b200.h WC_WIDE_REFSIZE_MAX
 
-    corrected: CUDA float64 [N][S] (bin-major).  Returns (indexes int32 [rows][refsize], distances float64
-    [rows][refsize]) on the same device; indexes are positions in the other-chromosome concatenation.
-    """
+
+def _topk_call(entry, corrected, chrom_bins, row_begin, row_end, refsize, out_idx, out_dist):
     _require_cuda(corrected, F64, "corrected")
     n, s = corrected.shape
     cb = np.ascontiguousarray(chrom_bins, dtype=np.int32)
@@ -29,11 +28,49 @@ def newref_topk(corrected, chrom_bins, row_begin, row_end, refsize, out_idx=None
     if out_dist is None:
         out_dist = _mem.empty((max(rows, 0), refsize), F64, like=corrected)
     ctx = _cabi.context(_mem.device_index(corrected))
-    rc = _cabi.lib().wc_newref_topk(ctx.handle, _ptr(corrected), n, s, cb.ctypes.data_as(ctypes.c_void_p), len(cb),
-                                    int(row_begin), int(row_end), int(refsize), _ptr(out_idx), _ptr(out_dist),
-                                    _stream_ptr(corrected))
+    rc = entry(ctx.handle, _ptr(corrected), n, s, cb.ctypes.data_as(ctypes.c_void_p), len(cb), int(row_begin), int(row_end),
+               int(refsize), _ptr(out_idx), _ptr(out_dist), _stream_ptr(corrected))
     _cabi.check(rc)
     return out_idx, out_dist
+
+
+def newref_topk(corrected, chrom_bins, row_begin, row_end, refsize, out_idx=None, out_dist=None):
+    """Reference-bin search for target rows [row_begin, row_end) (wisetools.py:364-398, 298-325), refsize 1..384.
+
+    corrected: CUDA float64 [N][S] (bin-major).  Returns (indexes int32 [rows][refsize], distances float64
+    [rows][refsize]) on the same device; indexes are positions in the other-chromosome concatenation.
+    """
+    return _topk_call(_cabi.lib().wc_newref_topk, corrected, chrom_bins, row_begin, row_end, refsize, out_idx, out_dist)
+
+
+def newref_topk_wide(corrected, chrom_bins, row_begin, row_end, refsize, out_idx=None, out_dist=None):
+    """The same search for refsize 1..WIDE_REFSIZE_MAX (wc_newref_topk_wide: exact distances of every pair, then a
+    select per row).  Same arguments and results as newref_topk."""
+    return _topk_call(_cabi.lib().wc_newref_topk_wide, corrected, chrom_bins, row_begin, row_end, refsize, out_idx,
+                      out_dist)
+
+
+def newref_search(corrected, chrom_bins, row_begin, row_end, refsize, device=0, out_idx=None, out_dist=None):
+    """The reference-bin search with the entry that serves `refsize`: wc_newref_topk up to NARROW_REFSIZE_MAX, the wide
+    search above.  corrected may be a device array (results on its device, of its kind) or a host numpy array (results
+    in numpy; `device` runs it).  Host input of a wide search is uploaded through _mem, so no PyTorch is needed."""
+    refsize = int(refsize)
+    if not 1 <= refsize <= WIDE_REFSIZE_MAX:
+        raise _cabi.WisecondorError("refsize must be between 1 and %d (got %d)" % (WIDE_REFSIZE_MAX, refsize))
+    if _mem.is_device(corrected):
+        fn = newref_topk if refsize <= NARROW_REFSIZE_MAX else newref_topk_wide
+        return fn(corrected, chrom_bins, row_begin, row_end, refsize, out_idx, out_dist)
+    if refsize <= NARROW_REFSIZE_MAX:
+        return newref_topk_host(corrected, chrom_bins, row_begin, row_end, refsize, device=device, out_idx=out_idx,
+                                out_dist=out_dist)
+    x = _mem.to_device(np.ascontiguousarray(corrected, dtype=np.float64), device)
+    idx, dist = newref_topk_wide(x, chrom_bins, row_begin, row_end, refsize)
+    idx, dist = _mem.to_host(idx), _mem.to_host(dist)
+    if out_idx is not None:
+        out_idx[...] = idx
+        out_dist[...] = dist
+        return out_idx, out_dist
+    return idx, dist
 
 
 def newref_topk_host(corrected, chrom_bins, row_begin, row_end, refsize, device=0, out_idx=None, out_dist=None):

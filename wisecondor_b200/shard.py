@@ -83,6 +83,9 @@ class ShardedSearch(object):
         self.full = torch.empty((world * self.rows_per, self.s), dtype=torch.float64, device=device)
         self.r0, self.r1 = row_shard(rank, world, self.n)            # search rows: the reference's getPart
         self.sym = None
+        if symmetric and self.k > _dev.NARROW_REFSIZE_MAX:
+            raise ValueError("the symmetric sharded search takes refsize up to %d (got %d): use row shards"
+                             % (_dev.NARROW_REFSIZE_MAX, self.k))
         if symmetric:        # block pairs instead of rows: this rank's bins are the blocks it owns (SymmetricShardedSearch)
             self.sym = SymmetricShardedSearch(self.n, self.k, rank, world, device, group=group)
             self.r0, self.r1 = self.sym.row0, max(self.sym.row0, self.sym.row1)
@@ -107,7 +110,7 @@ class ShardedSearch(object):
         if self.sym is not None:
             self.idx, self.dist = self.sym.run(x, chrom_bins)
         else:
-            self._dev.newref_topk(x, chrom_bins, self.r0, self.r1, self.k, self.idx, self.dist)
+            self._dev.newref_search(x, chrom_bins, self.r0, self.r1, self.k, out_idx=self.idx, out_dist=self.dist)
         self.h_idx.copy_(self.idx, non_blocking=True)
         self.h_dist.copy_(self.dist, non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()

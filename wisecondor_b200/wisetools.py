@@ -38,13 +38,13 @@ def getReference(correctedData, chromosomeBins, chromosomeBinSums, selectRefAmou
     if _mem.is_device(correctedData):
         if correctedData.shape[0] != bincount:
             raise ValueError("correctedData has %d bins, chromosomeBinSums says %d" % (correctedData.shape[0], bincount))
-        idx, dist = _dev.newref_topk(correctedData, bins, startNum, endNum, int(selectRefAmount))
+        idx, dist = _dev.newref_search(correctedData, bins, startNum, endNum, int(selectRefAmount))
         idx, dist = _mem.to_host(idx), _mem.to_host(dist)
     else:
         X = np.ascontiguousarray(correctedData, dtype=np.float64)
         if X.shape[0] != bincount:
             raise ValueError("correctedData has %d bins, chromosomeBinSums says %d" % (X.shape[0], bincount))
-        idx, dist = _dev.newref_topk_host(X, bins, startNum, endNum, int(selectRefAmount), device=dev)
+        idx, dist = _dev.newref_search(X, bins, startNum, endNum, int(selectRefAmount), device=dev)
     print('Time spent:', int(time.time() - timeStart), 'seconds')
     return idx, dist
 
